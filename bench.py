@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - headline benchmark of the Fast-SRGAN B200 engine (driver contract, see DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): generator-only 4x super-resolution, 180x320 -> 720x1280,
 batch 32 frames per GPU per step, L=8 residual blocks, F=64, synthetic frames, random-init weights.
@@ -13,7 +13,10 @@ One "step" = one pass of Generator.forward over one batch.  Metric: SR frames/s 
   roofline     : dominant kernel (the 64->256 upsampling conv at 360x640), timed per launch inside the
                  timed region with CUDA events on its launch stream (fsr_profile_* hooks).
   cpu_baseline : the oracle port of the reference generator on the host cores, bounded sample.
-  --impl reference : the reference CPU path (oracle port; /root/reference is Python and cannot travel).
+  --impl reference : the reference CPU path (the oracle port of the reference generator).
+  --dump-outputs DIR : after the timed steps, rank 0 writes what its last step returned to the caller, as float32
+          .npy files (56 MB in all): value's Generator.forward output (frame 0 in full + a seeded sample of the batch)
+          and e2e's uint8 frames (the same).  Inputs and weights are seeded, so two builds can be compared file by file.
 Multi-GPU: frames are independent -> one replica per rank, no data-path collective ("weak" scaling).
 """
 import argparse
@@ -95,31 +98,14 @@ def _host_threads():
 
 
 class _CpuGenerator:
-    """The reference's CPU implementation of the path: the UNMODIFIED reference model.py from git-ignored baseline/_ref/
-    (placed there by __graft_entry__.build() while /root/reference is mounted; it travels to the GPU box with the
-    snapshot) - kind "reference"; when that copy is absent, the oracle port of model.py:112-117 - kind "port"."""
+    """The reference's CPU implementation of the path, as the oracle port of model.py:112-117 - kind "port"."""
 
     def __init__(self):
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import srgan_oracle as O
         self.sd = O.make_generator_state(NF, NL, seed=1234)
-        ref_dir = os.path.join(ROOT, "baseline", "_ref")
         self.kind, self.what = "port", "oracle port of model.py:112-117 (oracle/srgan_oracle.py), fp32 oneDNN"
         self.fn = lambda x: O.generator_forward(self.sd, x)
-        if os.path.exists(os.path.join(ref_dir, "model.py")):
-            try:
-                sys.path.insert(0, ref_dir)
-                import types
-                import model as ref_model                       # the reference's own model.py, unmodified
-                g = ref_model.Generator(types.SimpleNamespace(n_filters=NF, n_layers=NL))
-                g.load_state_dict(self.sd)
-                g.eval()
-                self.fn, self.kind = g, "reference"
-                self.what = "unmodified reference model.py Generator.forward (baseline/_ref), fp32 oneDNN, eval/no_grad"
-            except Exception as exc:                            # torchvision missing etc.: say so, use the port
-                self.what += f" [baseline/_ref import failed: {exc!r}]"
-            finally:
-                sys.path.remove(ref_dir)
 
 
 def _cpu_setup():
@@ -164,8 +150,7 @@ def cpu_generator_fps(budget_s=20.0):
 
 
 def run_reference(args, rank, world):
-    """--impl reference: the reference's own CPU implementation of the path, rank 0 only: the unmodified reference
-    model.py from baseline/_ref when present (kind "reference"), else the oracle port (kind "port")."""
+    """--impl reference: the reference's CPU implementation of the path (the oracle port), rank 0 only."""
     if rank != 0:
         return
     O, sd = _cpu_setup()
@@ -221,6 +206,16 @@ def load_traffic():
     return {}
 
 
+DUMP_SAMPLE = 1 << 22
+
+
+def output_sample(name, t):
+    """{<name>_frame0: frame 0 in full, <name>_sample: DUMP_SAMPLE values of the whole tensor at seeded positions},
+    float32 host arrays; t is a caller's output, batch first."""
+    idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    return {f"{name}_frame0": t[0].float().cpu().numpy(), f"{name}_sample": t.reshape(-1)[idx.to(t.device)].float().cpu().numpy()}
+
+
 def _time_steps(fn, n, dev, dist):
     torch.cuda.synchronize()
     if dist is not None:
@@ -250,7 +245,7 @@ def bench_train_step(args, rank, world, dev, dist, lib):
     import warnings
     from fast_srgan_b200.trainer import Trainer
     ns = types.SimpleNamespace
-    steps = max(5, min(args.steps, 20))
+    steps = args.steps
     FLOPS_B64 = 2636e9                                 # SURVEY.md 8(a10)/(d): needed conv FLOPs of one step at batch 64
 
     def make(B, standalone):
@@ -375,7 +370,12 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the auxiliary GAN train-step measurement")
     ap.add_argument("--streams", type=int, default=int(os.environ.get("FSR_STREAMS", "1")),
                     help="sub-batches of the forward run concurrently on internal side streams (1 = single stream)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -446,6 +446,7 @@ def main():
         clocks = sampler.stop() if rank == 0 else None
         prof = read_profile(lib)
         lib.fsr_profile_enable_mask(0)
+        dumps = output_sample("sr", y) if args.dump_outputs else {}
     up1_flops = 2.0 * BATCH * (2 * H) * (2 * W) * 64 * 256 * 9
     # two upsampling convs per step: the 360x640 launches are the ones tagged with up1's FLOPs
     up1 = [ms for ms, fl in prof.get(L.K_CONV_UP, []) if abs(fl - up1_flops) < 1e-3 * up1_flops]
@@ -489,6 +490,8 @@ def main():
     e2e_loop(args.steps)
     torch.cuda.synchronize()
     wall_ms = (time.perf_counter() - wall0) * 1e3
+    if args.dump_outputs:
+        dumps.update(output_sample("sr_u8", h_out[(args.steps - 1) & 1]))
     barrier()
     e2e_ms = max_over_ranks(wall_ms)    # host-visible completion of the last D2H, max over ranks
     e2e_fps = world * BATCH * args.steps / (e2e_ms / 1e3)
@@ -553,6 +556,11 @@ def main():
         line["cpu_baseline"] = {"value": cfps, "unit": UNIT, "cores": cthreads, "kind": ckind, "sample": csample}
     if dist is not None:
         dist.destroy_process_group()
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     emit(line)
 
 

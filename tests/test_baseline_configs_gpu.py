@@ -5,7 +5,8 @@
               tests/golden/train_b64_golden.npz (oracle/make_golden_b64.py): losses, step-1 gradients per tensor,
               sign agreement of every parameter update of the trajectory
   f1          three pre-training steps (trainer.py:104-111) at batch 16 vs the same fixture
-  fixture     the reference's shipped checkpoint models/model.pt (tests/golden/checkpoint_golden.npz)
+  fixture     the reference's shipped checkpoint models/model.pt, conv weights int8 per output channel
+              (tests/golden/checkpoint_golden.npz, oracle/make_ckpt_golden.py)
 
 The gradient / update figures are printed per tensor and, when FSR_REPORT_DIR is set, written as a markdown report
 (committed as profiles/r02/grad_parity.md).
@@ -72,28 +73,28 @@ def test_generator_180x320_frame_vs_oracle(dt, tol):
 
 
 # ------------------------------------------------------------------------------------------- shipped checkpoint
-def _ckpt_state(ckpt):
-    return {k[3:]: torch.from_numpy(ckpt[k]) for k in ckpt.files if k.startswith("sd/")}     # keys keep `_orig_mod.`
-
-
 @pytest.mark.parametrize("dt,tol", [(torch.float32, 1e-3), (torch.float16, 6e-3), (torch.bfloat16, 6e-2)])
 def test_shipped_checkpoint_parity(ckpt, dt, tol):
-    """models/model.pt loaded the way inference.py:27-35 does (`_orig_mod.` keys), 90x160 anchor frame of SURVEY 8c,
-    against the output of the UNMODIFIED reference (fixture).  The trained weights amplify operand rounding through 17
-    stacked InstanceNorms (residual stream |x| up to 17): fp16 operands measure ~3e-3 here (SURVEY 0 predicted 3.2e-3),
-    bf16 ~3e-2; north_star's 1e-3 on this fixture needs the precise mode (compute_dtype=torch.float32: fp16 hi+lo
-    split operands, fp32 storage)."""
+    """models/model.pt (conv weights int8 per output channel) loaded the way inference.py:27-35 does (`_orig_mod.`
+    keys), 90x160 anchor frame of SURVEY 8c, against the output of the UNMODIFIED reference at the fixture's seeded
+    sample of output positions.  The trained weights amplify operand rounding through 17 stacked InstanceNorms
+    (residual stream |x| up to 17): fp16 operands measure ~3e-3 here (SURVEY 0 predicted 3.2e-3), bf16 ~3e-2;
+    north_star's 1e-3 on this fixture needs the precise mode (compute_dtype=torch.float32: fp16 hi+lo split
+    operands, fp32 storage)."""
+    import make_ckpt_golden as MC
     from fast_srgan_b200.model import Generator
     g = Generator(ns(n_filters=64, n_layers=8), compute_dtype=dt)
-    g.load_state_dict(_ckpt_state(ckpt))
+    g.load_state_dict(MC.state_dict(ckpt))                                      # keys keep `_orig_mod.`
     g = g.cuda().eval()
-    x = torch.from_numpy(ckpt["x0"])
     with torch.no_grad():
-        y = g(x.cuda()).cpu()
-    ref = torch.from_numpy(ckpt["y0"])
-    err = (y - ref).abs().max().item()
-    print(f"shipped checkpoint, 1x3x90x160, {dt}: max-abs vs reference {err:.3e}  mean-abs {(y - ref).abs().mean().item():.3e}")
-    assert y.shape == ref.shape and err <= tol
+        y = g(MC.anchor_input().cuda()).cpu()
+    assert y.shape == (1, 3, 360, 640)
+    got = y.reshape(-1)[MC.sample_idx(y.numel())]
+    ref = torch.from_numpy(ckpt["y_sample"])
+    err = (got - ref).abs().max().item()
+    print(f"shipped checkpoint, 1x3x90x160, {dt}: max-abs vs reference {err:.3e}  mean-abs {(got - ref).abs().mean().item():.3e}"
+          f"  ({ref.numel()} sampled outputs)")
+    assert err <= tol
 
 
 # ------------------------------------------------------------------------------------------- configs[2]
@@ -139,7 +140,7 @@ def _grad_table(title, nets, gold, prefix, S):
 def test_train_step_b64_three_steps_vs_fp64_oracle(gold64, dt, ltol):
     """BASELINE configs[2] (batch 64, 24x24 LR / 96x96 HR), three consecutive steps with persistent AdamW state:
     steps 1-2 run eagerly, step 3 is the captured CUDA graph.  Asserted: the four losses of every step against the
-    fp64 oracle; step-1 gradients per tensor (rel-L2 and cosine over a 16 K-element subsample, full-tensor norm ratio);
+    fp64 oracle; step-1 gradients per tensor (rel-L2 and cosine over a seeded 2 K-element subsample, full-tensor norm ratio);
     sign agreement of every parameter update."""
     import make_golden_b64 as MG
     tr = _trainer(dt)
